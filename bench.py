@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — headline benchmark of the quantized-linear hot path.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--bs 32] [--impl ours|reference] [--quick]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--bs 32] [--impl ours|reference] [--quick] [--dump-outputs DIR]
 
 Metric (BASELINE.json): tok/s of the Llama-3-8B int4 weight-only (tile_packed_to_4d, group_size=32) linear stack.
 One "step" = one pass of all 32 layers of quantized linears over a batch of `bs` tokens per GPU (decode: one token
@@ -39,6 +39,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 GROUP = 32
 # (hidden, intermediate, kv, layers): SURVEY §8 shape table.  Kept here (not imported from ao_b200) so that the
@@ -248,6 +249,8 @@ def run_ours(args):
         bcast_bytes = broadcast_packed_weights(model, src=0)  # the one collective of the whole job
         torch.cuda.synchronize()
 
+    dumps = {}
+
     def measure(bs, with_e2e=True, clocks=False):
         gen = torch.Generator(device=dev).manual_seed(1 + rank)
         x_static = (torch.randn(bs, hidden, device=dev, generator=gen)).to(torch.bfloat16)
@@ -257,6 +260,8 @@ def run_ours(args):
             sampler.start()
         ms = time_replays(graph, args.steps, args.warmup, barrier)
         clk = sampler.stop() if sampler else None
+        if args.dump_outputs:
+            dumps[f"int4_stack_bs{bs}"] = y_static.float().cpu().numpy()   # the last timed step's model output
         res = {"ms": ms, "launches": launches, "clocks": clk, "finite": bool(torch.isfinite(y_static.float()).all())}
         if with_e2e:
             # end-to-end: host buffers, H2D + D2H inside the timed region
@@ -278,15 +283,14 @@ def run_ours(args):
             res["ms_e2e"] = e2.elapsed_time(e3) / args.steps
             # eager (no graph) end-to-end, for reference
             e4, e5 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-            n_eager = max(1, min(args.steps, 5))
             e4.record()
             with torch.no_grad():
-                for _ in range(n_eager):
+                for _ in range(args.steps):
                     y = model(x_host.to(dev, non_blocking=True))
                     y_host.copy_(y, non_blocking=True)
             e5.record()
             barrier()
-            res["ms_eager"] = e4.elapsed_time(e5) / n_eager
+            res["ms_eager"] = e4.elapsed_time(e5) / args.steps
             res["h2d"], res["d2h"] = x_host.numel() * 2, y_host.numel() * 2
             res["ms"], res["ms_e2e"], res["ms_eager"] = max_over_ranks([res["ms"], res["ms_e2e"], res["ms_eager"]])
         else:
@@ -295,6 +299,8 @@ def run_ours(args):
 
     main = measure(args.bs, clocks=True)
     bs1 = measure(1) if args.bs != 1 else main
+    if args.dump_outputs and rank == 0:
+        write_dumps(args.dump_outputs, dumps)
 
     # ---- the kernel the reference calls on a GPU, same weights / chain / protocol / box --------------------
     gpu_ref = None
@@ -369,6 +375,28 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def write_dumps(out_dir, arrays):
+    """Write each output as out_dir/<name>.npy in float32.  Above DUMP_LIMIT bytes in all, an array keeps a fixed,
+    seeded sample of its rows (in order), so two runs with the same arguments write files that compare element for
+    element."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(arrays.items(), key=lambda kv: kv[1].nbytes)
+    budget = DUMP_LIMIT - 1024 * len(items)   # room for the .npy headers
+    for i, (name, a) in enumerate(items):
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        share = budget // (len(items) - i)
+        if a.nbytes > share:
+            keep = share // (a.nbytes // a.shape[0])
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        budget -= a.nbytes
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def gpu_reference_int4(model, hidden, batch_sizes, args, dev, barrier):
     """aten._weight_int4pack_mm (PyTorch-core tinygemm kernel; what Int4TilePackedTo4dTensor's handler calls at
     int4_tile_packed_to_4d_tensor.py:287) on OUR packed weights (the layouts are bit-identical, tests/test_int4_gpu.py),
@@ -415,7 +443,7 @@ def gpu_reference_int4(model, hidden, batch_sizes, args, dev, barrier):
 
     out = {"kernel": "aten._weight_int4pack_mm (torch " + torch.__version__ + ")",
            "protocol": "same packed weights, same dependent chain, CUDA-graph replays, CUDA events"}
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     for bs in batch_sizes:
         x = torch.randn(bs, hidden, device=dev).to(torch.bfloat16)
         rec = {}
@@ -525,7 +553,7 @@ def other_configs(args, dev, world, rank, barrier, max_over_ranks, peak):
     from ao_b200.prototype.mx_formats.inference_workflow import NVFP4WeightFloat8ActivationConfig
     from ao_b200.quantization import (Float8DynamicActivationFloat8WeightConfig, Int8DynamicActivationInt8WeightConfig, PerRow)
 
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     plans = []
     if world == 1:
         plans = [
@@ -795,7 +823,14 @@ if __name__ == "__main__":
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--quick", action="store_true", help="headline only: skip gpu_reference and the other configs")
     ap.add_argument("--no-fuse", action="store_true", help="7 launches per layer (q, k, v, gate, up not fused)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline stack's output of the last timed step at --bs and at "
+                         "bs=1 as DIR/int4_stack_bs<N>.npy (float32, seeded inputs, at most 64 MB in all)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if a.warmup < 3:
         a.warmup = 3
     if a.impl == "reference":
