@@ -112,8 +112,9 @@ def test_linear_full_size_vs_aten_and_linearity(ops, M, N, K):
     (700, 256, 2048, 256, False),
 ])
 def test_prefill_kernel_vs_oracle(ops, M, N, K, g, bias):
-    """M > 128 runs the prefill-shaped kernel (csrc/ts_prefill.cuh: 256-token tiles, weights dequantised once per
-    tile); same oracle, same 45 dB bar as the decode kernel, ragged token / feature tails included."""
+    """M > 128 at small N x K: below the prefill crossover (ts_prefill.cuh `worth_it`), so these run the decode kernel's
+    128-token variant over several token blocks (the prefill kernel itself: tests/test_kernel_paths_gpu.py); same
+    oracle, same 45 dB bar, ragged token / feature tails included."""
     o = _o()
     q, q_u8, sz = _mk_q(N, K, g, M * 5 + N)
     qd = ops.int4_pack_tile4d(q_u8, 8)
@@ -133,7 +134,10 @@ def test_prefill_kernel_vs_oracle(ops, M, N, K, g, bias):
 @pytest.mark.parametrize("M,N,K", [(512, 4096, 4096), (512, 4096, 14336), (300, 6144, 4096), (2048, 1024, 4096)])
 def test_prefill_full_size_vs_aten_and_properties(ops, M, N, K):
     """BASELINE layer shapes at prefill token counts (tiles split across CTAs by the stream-K walk): the reference's own
-    kernel, run-to-run determinism, one-hot exactness in every 256-token block, exact power-of-two scaling."""
+    kernel, run-to-run determinism, one-hot exactness in rows 0, 255, 256 and M - 1, exact power-of-two scaling.  All
+    four shapes are below the prefill crossover (fewer than 50 chunks of 128 x 256 x 128 per SM), so they run the
+    decode kernel's 128-token variant with several token blocks; the prefill kernel has its own tests in
+    tests/test_kernel_paths_gpu.py."""
     g = 32
     q, q_u8, sz = _mk_q(N, K, g, 11)
     qd = ops.int4_pack_tile4d(q_u8, 8)

@@ -190,7 +190,9 @@ def test_block_scaled_linears_vs_the_library_kernel(ops, M, N, K):
 
 @pytest.mark.parametrize("M,N,K,fp8_act", [(1, 256, 1024, False), (32, 4096, 4096, False), (7, 1024, 4096, True), (32, 8192, 8192, True),
                                            (64, 1024, 2048, False), (130, 512, 1024, True),
-                                           (512, 8192, 8192, True), (300, 1024, 4096, False)])  # M > 128: prefill kernel
+                                           (512, 8192, 8192, True), (300, 1024, 4096, False)])
+# of the M > 128 shapes only (512, 8192, 8192) is above the prefill crossover and runs the prefill kernel; (130, ...) and
+# (300, 1024, 4096) run the decode kernel's 128-token variant
 def test_nvfp4_weight_linear(ops, M, N, K, fp8_act):
     x = torch.randn(M, K, device="cuda").to(torch.bfloat16)
     w = (torch.randn(N, K, device="cuda") * 0.05).to(torch.bfloat16)
